@@ -3,7 +3,7 @@
 1e6 distinct keys, sum, 8 map → 8 reduce partitions, on one B200 (configs[1]); N>1 = the same
 per-GPU workload on every rank (weak scaling) with the combined rows exchanged by one all-to-all-v.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: create the shuffle, run the M map tasks
 (map-side combine: hash_agg_kernel), seal (merge + partition the combined rows).  `value` is
@@ -128,6 +128,42 @@ def traffic_lookup(kernel, rows_per_launch, table_slots):
     return None, None
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def u64_halves(a):
+    """(n, 2) float64 of [high 32 bits, low 32 bits]: exact, where a cast of a 64-bit key to float64 is not."""
+    import numpy as np
+    a = a.view(np.uint64)
+    return np.stack([(a >> np.uint64(32)).astype(np.float64), (a & np.uint64(0xFFFFFFFF)).astype(np.float64)], axis=1)
+
+
+def dump_outputs(out_dir, parts, suffix=""):
+    """Writes what the caller of the timed path receives from its last step: for each reduce partition this
+    rank owns (in order), the (key, sum) rows of Shuffle.reduce(r).  Rows are sorted by key inside each
+    partition, since their order there is unspecified, so that two builds compare row for row.
+    keys.npy / sums.npy: (n, 2) float64 u64 halves (u64_halves); partition_rows.npy: rows per partition.
+    Beyond DUMP_MAX_BYTES a fixed, seeded sample of rows is kept and sample_index.npy names them."""
+    import numpy as np
+    keys, sums = [], []
+    for k, c in parts:
+        o = np.argsort(k.view(np.uint64), kind="stable")
+        keys.append(k.view(np.uint64)[o])
+        sums.append(c.view(np.uint64)[o])
+    out = {"partition_rows": np.array([len(k) for k in keys], dtype=np.float64)}
+    keys, sums = np.concatenate(keys), np.concatenate(sums)
+    # 32 B of keys + sums and 8 B of sample index per row; 4 files with a .npy header of at most 256 B each
+    cap = (DUMP_MAX_BYTES - 4 * 256 - out["partition_rows"].nbytes) // 40
+    if len(keys) > cap:
+        idx = np.sort(np.random.default_rng(0).choice(len(keys), cap, replace=False))
+        keys, sums = keys[idx], sums[idx]
+        out["sample_index"] = idx.astype(np.float64)
+    out["keys"], out["sums"] = u64_halves(keys), u64_halves(sums)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -142,7 +178,11 @@ def main():
     ap.add_argument("--cpu-rows", type=float, default=None, help="rows per CPU step (default: full size for --impl reference if it fits in minutes, 1e8 for the in-run baseline)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's reduce_by_key result to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's result: use it with --impl ours")
     n_gpus = args.gpus
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -269,11 +309,16 @@ def main():
     # once across this rank's partitions and the sums add up to the sum of all values
     last = kept[-1]
     chk_keys, chk_sum = 0, 0
+    last_parts = []
     for r in vdist.owned_partitions(rank, world, n_red_global):
         k, c = last.reduce(r)
         chk_keys += len(k); chk_sum += int(c.sum(dtype=np.uint64))
+        last_parts.append((k, c))
     for sh in kept:
         sh.free()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_parts, f"_rank{rank}" if world > 1 else "")
+    del last_parts
     if world > 1:
         t = torch.tensor([ms_total, float(chk_keys), float(chk_sum % (1 << 52))], dtype=torch.float64, device=dev)
         tmax = t.clone(); tdist.all_reduce(tmax, op=tdist.ReduceOp.MAX)
