@@ -17,6 +17,8 @@
  *                             + ShuffleFetcher::fetch             src/shuffle/shuffle_fetcher.rs:16-119
  *   vb_join*               <- CoGroupedRdd::compute               src/rdd/co_grouped_rdd.rs:206-249
  *                             + PairRdd::join cross product       src/rdd/pair_rdd.rs:104-121
+ *   vb_cogroup*            <- PairRdd::cogroup                    src/rdd/pair_rdd.rs:123-155
+ *   vb_join_outer*         <- (absent from the reference: Spark's left/right/full outer joins)
  *   vb_shuffle_free        <- (the reference never evicts SHUFFLE_CACHE, src/env.rs:27)
  *   vb_slice               <- ParallelCollection::slice           src/rdd/parallel_collection_rdd.rs:116-145
  *   vb_shuffle_export_* / vb_shuffle_import
@@ -235,6 +237,34 @@ VB_API int32_t vb_shuffle_reduce(vb_shuf *s, uint32_t reduce_id, void *out_keys,
 VB_API int32_t vb_join_size(vb_shuf *left, vb_shuf *right, uint32_t reduce_id, uint64_t *n_out);
 VB_API int32_t vb_join(vb_shuf *left, vb_shuf *right, uint32_t reduce_id, void *out_k, void *out_v, void *out_w,
                        int32_t dst_loc);
+
+/* PairRdd::cogroup (src/rdd/pair_rdd.rs:123-155, co_grouped_rdd.rs:206-249) for reduce partition r
+ * of two sealed GROUP/COGROUP shuffles with the same n_reduce and key width.  Keys in union order:
+ * the left side's keys in its CSR order, then the right-only keys in the right CSR order.  Each
+ * key's values per side in input order; a key absent on a side has an empty list there.
+ * Argument checks, blocking and error codes as vb_join; 0 keys on a rank that does not own r.    */
+VB_API int32_t vb_cogroup_size(vb_shuf *left, vb_shuf *right, uint32_t reduce_id,
+                               uint64_t *n_keys, uint64_t *n_left_vals, uint64_t *n_right_vals);
+VB_API int32_t vb_cogroup(vb_shuf *left, vb_shuf *right, uint32_t reduce_id,
+                          void *out_keys,        /* n_keys */
+                          uint64_t *out_offs_l,  /* n_keys + 1, partition-local, [0] = 0 */
+                          void *out_vals_l,      /* n_left_vals */
+                          uint64_t *out_offs_r,  /* n_keys + 1 */
+                          void *out_vals_r,      /* n_right_vals */
+                          int32_t dst_loc);      /* VB_HOST | VB_DEVICE, as vb_join */
+
+/* Left / right / full outer join: absent from the reference; Spark semantics; parity unpinned.
+ * Rows of one key are contiguous, keys in the cogroup's union order.  A key with values on both
+ * sides gives `for v in vs { for w in ws }` (as vb_join); LEFT_OUTER adds (v, absent) for a
+ * left-only key, RIGHT_OUTER (absent, w) for a right-only key, FULL_OUTER both.  An absent value
+ * is written as 0 and its bit is clear in out_valid[i] (VB_JOIN_HAS_V | VB_JOIN_HAS_W on matched
+ * rows).  A bad kind is VB_ERR_INVALID; otherwise checks, blocking and codes as vb_join.        */
+enum vb_join_kind { VB_JOIN_LEFT_OUTER = 1, VB_JOIN_RIGHT_OUTER = 2, VB_JOIN_FULL_OUTER = 3 };
+enum vb_join_valid { VB_JOIN_HAS_V = 1, VB_JOIN_HAS_W = 2 };   /* bits of out_valid[i] */
+VB_API int32_t vb_join_outer_size(vb_shuf *left, vb_shuf *right, uint32_t reduce_id, int32_t kind, uint64_t *n_out);
+VB_API int32_t vb_join_outer(vb_shuf *left, vb_shuf *right, uint32_t reduce_id, int32_t kind,
+                             void *out_k, void *out_v, void *out_w, uint8_t *out_valid /* may be NULL */,
+                             int32_t dst_loc);
 
 /* ---- SURVEY §8(f) N1: bincode blobs — the payload format of SHUFFLE_CACHE ------------------------
  * The reference serialises every (map, reduce) bucket with bincode 1.2.1 defaults (src/dependency.rs:213-214:

@@ -4,6 +4,8 @@
 // behaviour as the reference for the calls on the path —
 //   Context::new / make_rdd / parallelize          src/context.rs:333-345,399-431
 //   PairRdd::group_by_key / reduce_by_key / join   src/rdd/pair_rdd.rs:35-52,54-80,104-121
+//   PairRdd::cogroup                               src/rdd/pair_rdd.rs:123-155
+//   left / right / full outer joins                (absent from the reference; Spark semantics, std::optional sides)
 //   Rdd::count_by_value / distinct / collect       src/rdd/rdd.rs:450-459,502-522,420-434
 //   Rdd::intersection / subtract                   src/rdd/rdd.rs:838-946
 // Rows are Vec<(K,V)> with K in {u64,i64,i32,u32} and V in {u64,i64,f64}; reduce_by_key takes a
@@ -12,6 +14,7 @@
 #pragma once
 #include <cstdint>
 #include <memory>
+#include <optional>
 #include <stdexcept>
 #include <string>
 #include <type_traits>
@@ -174,9 +177,74 @@ public:
         return out;
     }
 
+    // self.cogroup(other, num_splits).collect()  →  Vec<(K, (Vec<V>, Vec<W>))>; per partition the keys of self in its
+    // order, then the keys only `other` has; an empty Vec on the side that lacks a key
+    template <typename W>
+    std::vector<std::pair<K, std::pair<std::vector<V>, std::vector<W>>>> cogroup(const PairRddT<K, W> &other, size_t num_splits) const
+    {
+        auto a = detail::run_shuffle<K>(*sc_, keys_, &vals_, num_slices_, num_splits, detail::dtype<V>::code, VB_AGG_COGROUP);
+        auto b = detail::run_shuffle<K>(*sc_, other.keys_, &other.vals_, other.num_slices_, num_splits, detail::dtype<W>::code, VB_AGG_COGROUP);
+        std::vector<std::pair<K, std::pair<std::vector<V>, std::vector<W>>>> out;
+        for (uint32_t r = 0; r < num_splits; ++r) {
+            uint64_t nk = 0, nv = 0, nw = 0;
+            check(vb_cogroup_size(a.get(), b.get(), r, &nk, &nv, &nw));
+            std::vector<uint64_t> k(nk), ov(nk + 1), v(nv), ow(nk + 1), w(nw);
+            check(vb_cogroup(a.get(), b.get(), r, k.data(), ov.data(), v.data(), ow.data(), w.data(), VB_HOST));
+            for (uint64_t i = 0; i < nk; ++i) {
+                std::vector<V> vs;
+                std::vector<W> ws;
+                for (uint64_t j = ov[i]; j < ov[i + 1]; ++j) vs.push_back(detail::from_bits<V>(v[j]));
+                for (uint64_t j = ow[i]; j < ow[i + 1]; ++j) ws.push_back(detail::from_bits<W>(w[j]));
+                out.emplace_back(detail::from_bits<K>(k[i]), std::make_pair(std::move(vs), std::move(ws)));
+            }
+        }
+        return out;
+    }
+
+    // Spark's outer joins (absent from the reference): Vec<(K, (Option<V>, Option<W>))>, rows of a key contiguous
+    template <typename W>
+    std::vector<std::pair<K, std::pair<std::optional<V>, std::optional<W>>>> left_outer_join(const PairRddT<K, W> &other, size_t num_splits) const
+    {
+        return outer_join(other, num_splits, VB_JOIN_LEFT_OUTER);
+    }
+    template <typename W>
+    std::vector<std::pair<K, std::pair<std::optional<V>, std::optional<W>>>> right_outer_join(const PairRddT<K, W> &other, size_t num_splits) const
+    {
+        return outer_join(other, num_splits, VB_JOIN_RIGHT_OUTER);
+    }
+    template <typename W>
+    std::vector<std::pair<K, std::pair<std::optional<V>, std::optional<W>>>> full_outer_join(const PairRddT<K, W> &other, size_t num_splits) const
+    {
+        return outer_join(other, num_splits, VB_JOIN_FULL_OUTER);
+    }
+
     std::shared_ptr<Context> sc_;
     size_t num_slices_;
     std::vector<uint64_t> keys_, vals_;
+
+private:
+    template <typename W>
+    std::vector<std::pair<K, std::pair<std::optional<V>, std::optional<W>>>> outer_join(const PairRddT<K, W> &other, size_t num_splits, int kind) const
+    {
+        auto a = detail::run_shuffle<K>(*sc_, keys_, &vals_, num_slices_, num_splits, detail::dtype<V>::code, VB_AGG_COGROUP);
+        auto b = detail::run_shuffle<K>(*sc_, other.keys_, &other.vals_, other.num_slices_, num_splits, detail::dtype<W>::code, VB_AGG_COGROUP);
+        std::vector<std::pair<K, std::pair<std::optional<V>, std::optional<W>>>> out;
+        for (uint32_t r = 0; r < num_splits; ++r) {
+            uint64_t n = 0;
+            check(vb_join_outer_size(a.get(), b.get(), r, kind, &n));
+            std::vector<uint64_t> k(n), v(n), w(n);
+            std::vector<uint8_t> valid(n);
+            check(vb_join_outer(a.get(), b.get(), r, kind, k.data(), v.data(), w.data(), valid.data(), VB_HOST));
+            for (uint64_t i = 0; i < n; ++i) {
+                std::optional<V> ov;
+                std::optional<W> ow;
+                if (valid[i] & VB_JOIN_HAS_V) ov = detail::from_bits<V>(v[i]);
+                if (valid[i] & VB_JOIN_HAS_W) ow = detail::from_bits<W>(w[i]);
+                out.emplace_back(detail::from_bits<K>(k[i]), std::make_pair(ov, ow));
+            }
+        }
+        return out;
+    }
 };
 
 template <typename K>

@@ -15,6 +15,8 @@ pub const VB_AGG_GROUP: i32 = 0; pub const VB_AGG_SUM: i32 = 1; pub const VB_AGG
 pub const VB_AGG_MAX: i32 = 3; pub const VB_AGG_COUNT: i32 = 4; pub const VB_AGG_COGROUP: i32 = 5;
 pub const VB_PART_HASH_METRO64: i32 = 0;
 pub const VB_HOST: i32 = 0;
+pub const VB_JOIN_LEFT_OUTER: i32 = 1; pub const VB_JOIN_RIGHT_OUTER: i32 = 2; pub const VB_JOIN_FULL_OUTER: i32 = 3;
+pub const VB_JOIN_HAS_V: u8 = 1; pub const VB_JOIN_HAS_W: u8 = 2;
 
 #[link(name = "vega_b200")]
 extern "C" {
@@ -33,6 +35,14 @@ extern "C" {
     pub fn vb_join_size(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, n_out: *mut u64) -> i32;
     pub fn vb_join(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, out_k: *mut c_void, out_v: *mut c_void,
                    out_w: *mut c_void, dst_loc: i32) -> i32;
+    // CoGroupedRdd::compute (PairRdd::cogroup) and Spark's outer joins, one reduce partition
+    pub fn vb_cogroup_size(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, n_keys: *mut u64,
+                           n_left_vals: *mut u64, n_right_vals: *mut u64) -> i32;
+    pub fn vb_cogroup(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, out_keys: *mut c_void, out_offs_l: *mut u64,
+                      out_vals_l: *mut c_void, out_offs_r: *mut u64, out_vals_r: *mut c_void, dst_loc: i32) -> i32;
+    pub fn vb_join_outer_size(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, kind: i32, n_out: *mut u64) -> i32;
+    pub fn vb_join_outer(left: *mut vb_shuf, right: *mut vb_shuf, reduce_id: u32, kind: i32, out_k: *mut c_void,
+                         out_v: *mut c_void, out_w: *mut c_void, out_valid: *mut u8 /* may be null */, dst_loc: i32) -> i32;
     // N1: bincode blobs (the payload format of SHUFFLE_CACHE)
     pub fn vb_shuffle_reduce_blob_size(s: *mut vb_shuf, reduce_id: u32, n_bytes: *mut u64) -> i32;
     pub fn vb_shuffle_reduce_blob(s: *mut vb_shuf, reduce_id: u32, out_blob: *mut c_void, dst_loc: i32) -> i32;

@@ -6,7 +6,7 @@ interface for the path (rdd.py) plus the one-process-per-GPU exchange (dist.py).
 Importing works without a GPU (so the C ABI can be inspected); computing does not.
 """
 from ._lib import (LIB_PATH, SYMBOLS, VegaB200Error, lib)  # noqa: F401
-from .rdd import Context, Grouped, JoinedRdd, PairRdd, Rdd, Shuffle, ShuffledRdd, slice_starts  # noqa: F401
+from .rdd import Context, Grouped, JoinedRdd, OuterJoinedRdd, PairRdd, Rdd, Shuffle, ShuffledRdd, slice_starts  # noqa: F401
 
-__all__ = ["Context", "PairRdd", "Rdd", "Shuffle", "ShuffledRdd", "JoinedRdd", "Grouped", "slice_starts",
+__all__ = ["Context", "PairRdd", "Rdd", "Shuffle", "ShuffledRdd", "JoinedRdd", "OuterJoinedRdd", "Grouped", "slice_starts",
            "VegaB200Error", "lib", "LIB_PATH", "SYMBOLS"]

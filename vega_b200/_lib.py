@@ -17,6 +17,8 @@ VB_PART_HASH_METRO64, VB_PART_RANGE = 0, 1
 VB_HOST, VB_DEVICE, VB_DEVICE_BORROWED = 0, 1, 2
 VB_GEN_UNIFORM, VB_GEN_ZIPF, VB_GEN_UNIQUE = 0, 1, 2
 VB_XCHG_AUTO, VB_XCHG_NCCL, VB_XCHG_P2P = 0, 1, 2
+VB_JOIN_LEFT_OUTER, VB_JOIN_RIGHT_OUTER, VB_JOIN_FULL_OUTER = 1, 2, 3
+VB_JOIN_HAS_V, VB_JOIN_HAS_W = 1, 2
 VB_UNIQUE_ID_BYTES = 128
 
 KERNEL_CLASSES = ["hash_agg", "dict", "merge", "rp_hist", "rp_scan", "rp_scatter", "misc", "join"]
@@ -83,6 +85,10 @@ SYMBOLS = {
     "vb_shuffle_reduce": (_i32, [_vp, _u32, _vp, _vp, _vp, _vp, _i32]),
     "vb_join_size": (_i32, [_vp, _vp, _u32, _pu64]),
     "vb_join": (_i32, [_vp, _vp, _u32, _vp, _vp, _vp, _i32]),
+    "vb_cogroup_size": (_i32, [_vp, _vp, _u32, _pu64, _pu64, _pu64]),
+    "vb_cogroup": (_i32, [_vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _i32]),
+    "vb_join_outer_size": (_i32, [_vp, _vp, _u32, _i32, _pu64]),
+    "vb_join_outer": (_i32, [_vp, _vp, _u32, _i32, _vp, _vp, _vp, _vp, _i32]),
     "vb_shuffle_reduce_blob_size": (_i32, [_vp, _u32, _pu64]),
     "vb_shuffle_reduce_blob": (_i32, [_vp, _u32, _vp, _i32]),
     "vb_shuffle_map_blob": (_i32, [_vp, _u32, _vp, _u64, _i32]),

@@ -277,6 +277,16 @@ struct JoinPlan {
     u32 *match = nullptr;
 };
 
+// cogroup / outer joins of one partition: the union of both key sets (see cogroup_probe_kernel)
+struct CogroupPlan {
+    u32 nl = 0, nro = 0;       // left keys of the partition, right-only keys
+    u32 *match = nullptr;      // [nl] right dense id of each left key, or CG_NONE
+    u32 *ronly = nullptr;      // [nro] dense ids of the right-only keys, in right CSR order
+    int kind = 0;              // outer-join kind whose row positions are cached (0 = none yet)
+    u64 rows = 0;
+    u64 *rowpos = nullptr;     // [nl + nro] exclusive scan of the output rows per union key under `kind`
+};
+
 struct vb_shuf {
     vb_ctx *ctx = nullptr;
     u64 id = 0;
@@ -327,6 +337,7 @@ struct vb_shuf {
     u32 dict_log_cap = 0;
     u32 *dense_of_slot = nullptr;
     std::map<std::pair<const vb_shuf *, u32>, JoinPlan> join_plans;
+    std::map<std::pair<u64, u32>, CogroupPlan> cg_plans;   // by (right side's uid, reduce_id): kept from *_size to the fetch
     // COGROUP shuffles are grouped lazily: seal keeps the (owned) rows; the CSR is built by the first reduce call
     // (cogroup materialisation), or — if a join comes first — only for the keys that occur on BOTH sides.
     u64 uid = 0;                                   // process-unique id (cache key that survives pointer reuse)
@@ -2718,14 +2729,11 @@ __global__ void __launch_bounds__(CP_THREADS) compact_count_kernel(const unsigne
     __syncthreads();
     if (threadIdx.x == 0) { u32 t = 0; for (int w = 0; w < CP_THREADS / 32; ++w) t += ws[w]; block_cnt[blockIdx.x] = t; }
 }
-__global__ void __launch_bounds__(CP_THREADS)
-compact_scatter_kernel(const unsigned char *__restrict__ match, u64 n, const u64 *__restrict__ block_off, const u64 *__restrict__ keys,
-                       const u64 *__restrict__ vals, u64 *__restrict__ out_keys, u64 *__restrict__ out_vals)
+// this thread's CP_ITEMS flags (m) and the output index of its first flagged row
+__device__ __forceinline__ u64 compact_first_out(const unsigned char *__restrict__ match, u64 n, const u64 *__restrict__ block_off, u64 base,
+                                                 unsigned char (&m)[CP_ITEMS], u32 *ws)
 {
-    __shared__ u32 ws[CP_THREADS / 32];
     const u32 tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    const u64 base = (u64)blockIdx.x * CP_TILE + (u64)tid * CP_ITEMS;
-    unsigned char m[CP_ITEMS];
     u32 c = 0;
 #pragma unroll
     for (int i = 0; i < CP_ITEMS; ++i) { m[i] = (base + i < n) ? match[base + i] : 0; c += m[i]; }
@@ -2736,21 +2744,41 @@ compact_scatter_kernel(const unsigned char *__restrict__ match, u64 n, const u64
     __syncthreads();
     u32 wbase = 0;
     for (u32 w = 0; w < warp; ++w) wbase += ws[w];
-    u64 o = block_off[blockIdx.x] + wbase + incl - c;
+    return block_off[blockIdx.x] + wbase + incl - c;
+}
+__global__ void __launch_bounds__(CP_THREADS)
+compact_scatter_kernel(const unsigned char *__restrict__ match, u64 n, const u64 *__restrict__ block_off, const u64 *__restrict__ keys,
+                       const u64 *__restrict__ vals, u64 *__restrict__ out_keys, u64 *__restrict__ out_vals)
+{
+    __shared__ u32 ws[CP_THREADS / 32];
+    const u64 base = (u64)blockIdx.x * CP_TILE + (u64)threadIdx.x * CP_ITEMS;
+    unsigned char m[CP_ITEMS];
+    u64 o = compact_first_out(match, n, block_off, base, m, ws);
 #pragma unroll
     for (int i = 0; i < CP_ITEMS; ++i)
         if (m[i]) { out_keys[o] = keys[base + i]; if (out_vals) out_vals[o] = vals ? vals[base + i] : 0ull; ++o; }
 }
+// out[j] = id_base + i for the j-th flagged i
+__global__ void __launch_bounds__(CP_THREADS)
+compact_ids_kernel(const unsigned char *__restrict__ match, u64 n, const u64 *__restrict__ block_off, u32 id_base, u32 *__restrict__ out)
+{
+    __shared__ u32 ws[CP_THREADS / 32];
+    const u64 base = (u64)blockIdx.x * CP_TILE + (u64)threadIdx.x * CP_ITEMS;
+    unsigned char m[CP_ITEMS];
+    u64 o = compact_first_out(match, n, block_off, base, m, ws);
+#pragma unroll
+    for (int i = 0; i < CP_ITEMS; ++i)
+        if (m[i]) out[o++] = id_base + (u32)(base + i);
+}
 
 static int exclusive_scan_u64(vb_shuf *s, const u64 *in, u64 *out, u64 n, u64 *d_total);
 
-static int compact_rows(vb_shuf *s, const u64 *keys, const u64 *vals, u64 n, const unsigned char *match, DevBuf &ok, DevBuf &ov, u64 *m_out)
+// first half of a stable compaction: flagged rows per tile, scanned into tile offsets (off), and their total (m_out)
+static int compact_offsets(vb_shuf *s, const unsigned char *match, u64 n, DevBuf &off, u64 *m_out)
 {
     vb_ctx *c = s->ctx;
-    *m_out = 0;
-    if (n == 0) return VB_OK;
     const u64 blocks = (n + CP_TILE - 1) / CP_TILE;
-    DevBuf cnt(c), off(c), tot(c);
+    DevBuf cnt(c), tot(c);
     TRY(cnt.alloc(blocks * 8)); TRY(off.alloc(blocks * 8)); TRY(tot.alloc(8));
     {
         KLaunch kl(s, K_JOIN);
@@ -2758,17 +2786,44 @@ static int compact_rows(vb_shuf *s, const u64 *keys, const u64 *vals, u64 n, con
         TRY(kl.done("compact_count_kernel"));
     }
     TRY(exclusive_scan_u64(s, cnt.as<u64>(), off.as<u64>(), blocks, tot.as<u64>()));
-    u64 m = 0;
     CU(cudaMemcpyAsync(c->h_scratch, tot.p, 8, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
-    m = *(u64 *)c->h_scratch;
+    *m_out = *(u64 *)c->h_scratch;
+    return VB_OK;
+}
+
+static int compact_rows(vb_shuf *s, const u64 *keys, const u64 *vals, u64 n, const unsigned char *match, DevBuf &ok, DevBuf &ov, u64 *m_out)
+{
+    vb_ctx *c = s->ctx;
+    *m_out = 0;
+    if (n == 0) return VB_OK;
+    DevBuf off(c);
+    u64 m = 0;
+    TRY(compact_offsets(s, match, n, off, &m));
     *m_out = m;
     if (m == 0) return VB_OK;
     TRY(ok.alloc(m * 8));
     TRY(ov.alloc(m * 8));
     KLaunch kl(s, K_JOIN);
-    compact_scatter_kernel<<<(unsigned)blocks, CP_THREADS, 0, c->stream>>>(match, n, off.as<u64>(), keys, vals, ok.as<u64>(), ov.as<u64>());
+    compact_scatter_kernel<<<(unsigned)((n + CP_TILE - 1) / CP_TILE), CP_THREADS, 0, c->stream>>>(match, n, off.as<u64>(), keys, vals, ok.as<u64>(), ov.as<u64>());
     return kl.done("compact_scatter_kernel");
+}
+
+// the flagged indices i of [0, n), as id_base + i, in order (stable compaction)
+static int compact_ids(vb_shuf *s, const unsigned char *flag, u64 n, u32 id_base, DevBuf &out, u64 *m_out)
+{
+    vb_ctx *c = s->ctx;
+    *m_out = 0;
+    if (n == 0) return VB_OK;
+    DevBuf off(c);
+    u64 m = 0;
+    TRY(compact_offsets(s, flag, n, off, &m));
+    *m_out = m;
+    if (m == 0) return VB_OK;
+    TRY(out.alloc(m * 4));
+    KLaunch kl(s, K_JOIN);
+    compact_ids_kernel<<<(unsigned)((n + CP_TILE - 1) / CP_TILE), CP_THREADS, 0, c->stream>>>(flag, n, off.as<u64>(), id_base, out.as<u32>());
+    return kl.done("compact_ids_kernel");
 }
 
 static vb_shuf *make_internal_like(const vb_shuf *s)
@@ -3242,6 +3297,258 @@ extern "C" int32_t vb_join(vb_shuf *l, vb_shuf *r, uint32_t rid, void *out_k, vo
 }
 
 // ---------------------------------------------------------------------------------------------
+// cogroup and outer joins (PairRdd::cogroup, pair_rdd.rs:123-155 / co_grouped_rdd.rs:206-249; the outer joins are
+// Spark's).  Both need every key of a side, so both sides are grouped completely (no semi-join filter).  Per
+// partition: probe the right dictionary with the left keys (match + "seen" flags), compact the unseen right keys,
+// then either lay out both value lists in union order (cogroup) or expand the rows an outer join keeps.
+// ---------------------------------------------------------------------------------------------
+static void free_cogroup_plan(vb_ctx *c, CogroupPlan &p)
+{
+    dev_free(c, p.match); dev_free(c, p.ronly); dev_free(c, p.rowpos);
+    p = CogroupPlan();
+}
+
+static int cogroup_plan(vb_shuf *l, vb_shuf *r, u32 rid, CogroupPlan **out)
+{
+    vb_ctx *c = l->ctx;
+    const auto key = std::make_pair(r->uid, rid);
+    auto it = l->cg_plans.find(key);
+    if (it != l->cg_plans.end()) { *out = &it->second; return VB_OK; }
+    const u64 lb = l->bucket_off[rid], rb = r->bucket_off[rid];
+    const u32 nl = (u32)(l->bucket_off[rid + 1] - lb), nr = (u32)(r->bucket_off[rid + 1] - rb);
+    DevBuf match(c), ronly(c);
+    u64 nro = 0;
+    if (nl) {
+        TRY(match.alloc((u64)nl * 4));
+        if (!nr) CU(cudaMemsetAsync(match.p, 0xFF, (u64)nl * 4, c->stream));
+    }
+    if (nr) {
+        DevBuf flag(c);
+        TRY(flag.alloc(nr));
+        CU(cudaMemsetAsync(flag.p, 1, nr, c->stream));
+        if (nl) {
+            KLaunch kl(l, K_JOIN);
+            cogroup_probe_kernel<<<(nl + 255) / 256, 256, 0, c->stream>>>(l->res_keys, (u32)lb, nl, table_at(r->dict, r->dict_log_cap),
+                                                                           r->dense_of_slot, (u32)rb, (u32)rb + nr, match.as<u32>(),
+                                                                           flag.as<unsigned char>());
+            TRY(kl.done("cogroup_probe_kernel"));
+        }
+        TRY(compact_ids(l, flag.as<unsigned char>(), nr, (u32)rb, ronly, &nro));
+    }
+    CogroupPlan p;
+    p.nl = nl;
+    p.nro = (u32)nro;
+    p.match = (u32 *)match.release();
+    p.ronly = (u32 *)ronly.release();
+    *out = &l->cg_plans.emplace(key, p).first->second;
+    return VB_OK;
+}
+
+// row positions of an outer join of `kind` over the plan's union keys (cached for the fetch that follows a size call)
+static int cogroup_rows(vb_shuf *l, vb_shuf *r, u32 rid, CogroupPlan *p, int kind)
+{
+    if (p->kind == kind) return VB_OK;
+    vb_ctx *c = l->ctx;
+    dev_free(c, p->rowpos);
+    p->rowpos = nullptr;
+    p->rows = 0;
+    p->kind = 0;
+    const u32 nu = p->nl + p->nro;
+    if (nu) {
+        DevBuf cnt(c), pos(c), tot(c);
+        TRY(cnt.alloc((u64)nu * 8)); TRY(pos.alloc((u64)nu * 8)); TRY(tot.alloc(8));
+        {
+            KLaunch kl(l, K_JOIN);
+            cogroup_count_kernel<<<(nu + 255) / 256, 256, 0, c->stream>>>(p->nl, nu, (u32)l->bucket_off[rid], l->res_offs, p->match, p->ronly,
+                                                                          r->res_offs, kind, nullptr, nullptr, cnt.as<u64>());
+            TRY(kl.done("cogroup_count_kernel"));
+        }
+        TRY(exclusive_scan_u64(l, cnt.as<u64>(), pos.as<u64>(), nu, tot.as<u64>()));
+        CU(cudaMemcpyAsync(c->h_scratch, tot.p, 8, cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        p->rows = *(u64 *)c->h_scratch;
+        p->rowpos = (u64 *)pos.release();
+    }
+    p->kind = kind;
+    return VB_OK;
+}
+
+// both sides grouped completely (caller holds c->mu)
+static int cogroup_sides(vb_shuf *l, vb_shuf *r)
+{
+    TRY(ensure_grouped(l));
+    return ensure_grouped(r);
+}
+
+static void drop_cogroup_plan(vb_shuf *l, vb_shuf *r, u32 rid)
+{
+    auto it = l->cg_plans.find(std::make_pair(r->uid, rid));
+    if (it == l->cg_plans.end()) return;
+    free_cogroup_plan(l->ctx, it->second);
+    l->cg_plans.erase(it);
+}
+
+extern "C" int32_t vb_cogroup_size(vb_shuf *l, vb_shuf *r, uint32_t rid, uint64_t *n_keys, uint64_t *n_left_vals, uint64_t *n_right_vals)
+{
+    TRY(join_check(l, r, rid));
+    std::lock_guard<std::mutex> lk(l->ctx->mu);
+    CU(cudaSetDevice(l->ctx->device));
+    TRY(cogroup_sides(l, r));
+    CogroupPlan *p = nullptr;
+    TRY(cogroup_plan(l, r, rid, &p));
+    if (n_keys) *n_keys = (u64)p->nl + p->nro;
+    if (n_left_vals) *n_left_vals = l->val_off[rid + 1] - l->val_off[rid];
+    if (n_right_vals) *n_right_vals = r->val_off[rid + 1] - r->val_off[rid];
+    return VB_OK;
+}
+
+// the caller's buffer when it is device memory, else a temporary device buffer copied out at the end
+static int cogroup_target(vb_ctx *c, void *dst, int dst_loc, DevBuf &tmp, u64 bytes, void **out)
+{
+    if (dst_loc == VB_DEVICE) { *out = dst; return VB_OK; }
+    TRY(tmp.alloc(bytes));
+    *out = tmp.p;
+    return VB_OK;
+}
+
+static int cogroup_fetch(vb_shuf *l, vb_shuf *r, u32 rid, const CogroupPlan *p, void *out_keys, uint64_t *out_offs_l, void *out_vals_l,
+                         uint64_t *out_offs_r, void *out_vals_r, int32_t dst_loc)
+{
+    vb_ctx *c = l->ctx;
+    const u32 nl = p->nl, nu = p->nl + p->nro;
+    const u64 lb = l->bucket_off[rid];
+    const u64 lv0 = l->val_off[rid], nlv = l->val_off[rid + 1] - lv0;
+    const u64 nrv = r->val_off[rid + 1] - r->val_off[rid];
+    if (nu == 0) {
+        const u64 zero = 0;
+        for (uint64_t *o : {out_offs_l, out_offs_r})
+            if (o) CU(cudaMemcpyAsync(o, &zero, 8, dst_loc == VB_HOST ? cudaMemcpyHostToHost : cudaMemcpyHostToDevice, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        return VB_OK;
+    }
+    if (!out_keys || !out_offs_l || !out_offs_r || (nlv && !out_vals_l) || (nrv && !out_vals_r))
+        return set_err(VB_ERR_INVALID, "NULL output with %u keys to write", nu);
+    DevBuf cl(c), cr(c), bk(c), bol(c), bor(c), bvr(c);
+    void *dk = nullptr, *dol = nullptr, *dor = nullptr, *dvr = nullptr;
+    TRY(cogroup_target(c, out_keys, dst_loc, bk, (u64)nu * 8, &dk));
+    TRY(cogroup_target(c, out_offs_l, dst_loc, bol, ((u64)nu + 1) * 8, &dol));
+    TRY(cogroup_target(c, out_offs_r, dst_loc, bor, ((u64)nu + 1) * 8, &dor));
+    TRY(cogroup_target(c, out_vals_r, dst_loc, bvr, nrv * 8, &dvr));
+    // value counts per union key, scanned into the two offset arrays (offs[nu] = the side's value count)
+    TRY(cl.alloc((u64)nu * 8)); TRY(cr.alloc((u64)nu * 8));
+    {
+        KLaunch kl(l, K_JOIN);
+        cogroup_count_kernel<<<(nu + 255) / 256, 256, 0, c->stream>>>(nl, nu, (u32)lb, l->res_offs, p->match, p->ronly, r->res_offs, 0,
+                                                                      cl.as<u64>(), cr.as<u64>(), nullptr);
+        TRY(kl.done("cogroup_count_kernel"));
+    }
+    TRY(exclusive_scan_u64(l, cl.as<u64>(), (u64 *)dol, nu, (u64 *)dol + nu));
+    TRY(exclusive_scan_u64(l, cr.as<u64>(), (u64 *)dor, nu, (u64 *)dor + nu));
+    // union keys: the left key slice, then the right-only keys
+    if (nl) CU(cudaMemcpyAsync(dk, l->res_keys + lb, (u64)nl * 8, cudaMemcpyDeviceToDevice, c->stream));
+    if (p->nro) {
+        KLaunch kl(l, K_JOIN);
+        cogroup_keys_kernel<<<(p->nro + 255) / 256, 256, 0, c->stream>>>(p->ronly, p->nro, r->res_keys, (u64 *)dk + nl);
+        TRY(kl.done("cogroup_keys_kernel"));
+    }
+    // right values: segmented gather in union order
+    if (nrv) {
+        KLaunch kl(l, K_JOIN);
+        const u64 blocks = std::min<u64>((nrv + 255) / 256, (u64)c->sm_count * 8);
+        cogroup_gather_right_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>((const u64 *)dor, nu, nrv, nl, p->match, p->ronly, r->res_offs,
+                                                                             r->res_vals, (u64 *)dvr);
+        TRY(kl.done("cogroup_gather_right_kernel"));
+    }
+    // left values: the partition's left CSR is already in union order
+    TRY(copy_out(l, out_vals_l, l->res_vals ? l->res_vals + lv0 : nullptr, nlv * 8, dst_loc));
+    if (dst_loc == VB_HOST) {
+        TRY(copy_out(l, out_keys, dk, (u64)nu * 8, VB_HOST));
+        TRY(copy_out(l, out_offs_l, dol, ((u64)nu + 1) * 8, VB_HOST));
+        TRY(copy_out(l, out_offs_r, dor, ((u64)nu + 1) * 8, VB_HOST));
+        TRY(copy_out(l, out_vals_r, dvr, nrv * 8, VB_HOST));
+    }
+    CU(cudaStreamSynchronize(c->stream));
+    return VB_OK;
+}
+
+extern "C" int32_t vb_cogroup(vb_shuf *l, vb_shuf *r, uint32_t rid, void *out_keys, uint64_t *out_offs_l, void *out_vals_l,
+                              uint64_t *out_offs_r, void *out_vals_r, int32_t dst_loc)
+{
+    TRY(join_check(l, r, rid));
+    if (dst_loc != VB_HOST && dst_loc != VB_DEVICE) return set_err(VB_ERR_INVALID, "bad dst_loc");
+    vb_ctx *c = l->ctx;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CU(cudaSetDevice(c->device));
+    TRY(cogroup_sides(l, r));
+    CogroupPlan *p = nullptr;
+    TRY(cogroup_plan(l, r, rid, &p));
+    const int rc = cogroup_fetch(l, r, rid, p, out_keys, out_offs_l, out_vals_l, out_offs_r, out_vals_r, dst_loc);
+    cudaStreamSynchronize(c->stream);
+    drop_cogroup_plan(l, r, rid);
+    return rc;
+}
+
+static bool outer_kind_ok(int32_t kind) { return kind == VB_JOIN_LEFT_OUTER || kind == VB_JOIN_RIGHT_OUTER || kind == VB_JOIN_FULL_OUTER; }
+
+extern "C" int32_t vb_join_outer_size(vb_shuf *l, vb_shuf *r, uint32_t rid, int32_t kind, uint64_t *n_out)
+{
+    TRY(join_check(l, r, rid));
+    if (!outer_kind_ok(kind)) return set_err(VB_ERR_INVALID, "bad outer join kind %d", kind);
+    if (!n_out) return set_err(VB_ERR_INVALID, "n_out is NULL");
+    std::lock_guard<std::mutex> lk(l->ctx->mu);
+    CU(cudaSetDevice(l->ctx->device));
+    TRY(cogroup_sides(l, r));
+    CogroupPlan *p = nullptr;
+    TRY(cogroup_plan(l, r, rid, &p));
+    TRY(cogroup_rows(l, r, rid, p, kind));
+    *n_out = p->rows;
+    return VB_OK;
+}
+
+extern "C" int32_t vb_join_outer(vb_shuf *l, vb_shuf *r, uint32_t rid, int32_t kind, void *out_k, void *out_v, void *out_w,
+                                 uint8_t *out_valid, int32_t dst_loc)
+{
+    TRY(join_check(l, r, rid));
+    if (!outer_kind_ok(kind)) return set_err(VB_ERR_INVALID, "bad outer join kind %d", kind);
+    if (dst_loc != VB_HOST && dst_loc != VB_DEVICE) return set_err(VB_ERR_INVALID, "bad dst_loc");
+    vb_ctx *c = l->ctx;
+    std::lock_guard<std::mutex> lk(c->mu);
+    CU(cudaSetDevice(c->device));
+    TRY(cogroup_sides(l, r));
+    CogroupPlan *p = nullptr;
+    TRY(cogroup_plan(l, r, rid, &p));
+    int rc = cogroup_rows(l, r, rid, p, kind);
+    const u64 total = p->rows;
+    if (rc == VB_OK && total) {
+        if (!out_k || !out_v || !out_w) rc = set_err(VB_ERR_INVALID, "NULL output with %llu rows to write", (unsigned long long)total);
+        DevBuf bk(c), bv(c), bw(c), bvalid(c);
+        void *dk = nullptr, *dv = nullptr, *dw = nullptr, *dvalid = nullptr;
+        if (rc == VB_OK) rc = cogroup_target(c, out_k, dst_loc, bk, total * 8, &dk);
+        if (rc == VB_OK) rc = cogroup_target(c, out_v, dst_loc, bv, total * 8, &dv);
+        if (rc == VB_OK) rc = cogroup_target(c, out_w, dst_loc, bw, total * 8, &dw);
+        if (rc == VB_OK && out_valid) rc = cogroup_target(c, out_valid, dst_loc, bvalid, total, &dvalid);
+        if (rc == VB_OK) {
+            KLaunch kl(l, K_JOIN);
+            const u64 blocks = std::min<u64>((total + 255) / 256, (u64)c->sm_count * 8);
+            outer_expand_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(p->rowpos, p->nl + p->nro, total, p->nl, (u32)l->bucket_off[rid],
+                                                                         l->res_keys, l->res_offs, l->res_vals, p->match, p->ronly,
+                                                                         r->res_keys, r->res_offs, r->res_vals, (u64 *)dk, (u64 *)dv,
+                                                                         (u64 *)dw, (unsigned char *)dvalid);
+            rc = kl.done("outer_expand_kernel");
+        }
+        if (rc == VB_OK && dst_loc == VB_HOST) {
+            rc = copy_out(l, out_k, dk, total * 8, VB_HOST);
+            if (rc == VB_OK) rc = copy_out(l, out_v, dv, total * 8, VB_HOST);
+            if (rc == VB_OK) rc = copy_out(l, out_w, dw, total * 8, VB_HOST);
+            if (rc == VB_OK && out_valid) rc = copy_out(l, out_valid, dvalid, total, VB_HOST);
+        }
+        cudaStreamSynchronize(c->stream);
+    }
+    drop_cogroup_plan(l, r, rid);
+    return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
 // free / stats
 // ---------------------------------------------------------------------------------------------
 extern "C" int32_t vb_shuffle_free(vb_shuf *s)
@@ -3263,6 +3570,7 @@ extern "C" int32_t vb_shuffle_free(vb_shuf *s)
         dev_free(c, s->res_keys); dev_free(c, s->res_comb); dev_free(c, s->res_offs); dev_free(c, s->res_vals);
         dev_free(c, s->dict); dev_free(c, s->dense_of_slot);
         for (auto &kv : s->join_plans) { dev_free(c, kv.second.pos); dev_free(c, kv.second.match); }
+        for (auto &kv : s->cg_plans) free_cogroup_plan(c, kv.second);
         free_lazy_rows(s);
         cudaStreamSynchronize(c->stream);
     }

@@ -1240,6 +1240,123 @@ __global__ void join_expand_kernel(const u64 *__restrict__ pos /*[nl] exclusive*
 }
 
 // ---------------------------------------------------------------------------------------------
+// cogroup / outer joins (CoGroupedRdd::compute, co_grouped_rdd.rs:206-249): the union of the key sets of one
+// partition, in union order — first the nl left keys in left CSR order (union key u is left key lb + u, match[u]
+// its right dense id or CG_NONE), then the right keys no left key matched, in right CSR order (ronly[u - nl]).
+// ---------------------------------------------------------------------------------------------
+constexpr u32 CG_NONE = 0xFFFFFFFFu;
+enum : int { CG_LEFT = 1, CG_RIGHT = 2 };   // the sides an outer join keeps when the other one is empty (VB_JOIN_* bits)
+
+// join_probe_kernel for one partition, plus: the right key it hits is no longer right-only (ronly_flag[m - rb] = 0)
+__global__ void cogroup_probe_kernel(const u64 *__restrict__ lkeys, u32 lb, u32 nl, Table rtab, const u32 *__restrict__ r_dense,
+                                     u32 rb, u32 re, u32 *__restrict__ match, unsigned char *__restrict__ ronly_flag)
+{
+    const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= nl) return;
+    const u32 s = table_find(rtab, lkeys[lb + j]);
+    u32 m = CG_NONE;
+    if (s != 0xFFFFFFFFu) {
+        m = r_dense[s];
+        if (m >= rb && m < re) ronly_flag[m - rb] = 0;
+        else m = CG_NONE;
+    }
+    match[j] = m;
+}
+
+// value counts of union key u on both sides and its right dense id (CG_NONE: no right values)
+VB_D void cogroup_key(u32 u, u32 nl, u32 lb, const u64 *__restrict__ loffs, const u32 *__restrict__ match,
+                      const u32 *__restrict__ ronly, const u64 *__restrict__ roffs, u64 &lc, u64 &rc, u32 &m)
+{
+    if (u < nl) { lc = loffs[lb + u + 1] - loffs[lb + u]; m = match[u]; }
+    else { lc = 0; m = ronly[u - nl]; }
+    rc = m != CG_NONE ? roffs[m + 1] - roffs[m] : 0;
+}
+
+// largest u < nu with pos[u] <= o (union keys without output share pos with the next one)
+VB_D u32 cogroup_owner(const u64 *__restrict__ pos, u32 nu, u64 o)
+{
+    u32 lo = 0, hi = nu;
+    while (hi - lo > 1) {
+        const u32 mid = (lo + hi) >> 1;
+        if (pos[mid] <= o) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// per union key: left / right value counts (cnt_l / cnt_r, may be NULL) and output rows under an outer `kind` (cnt_rows, may be NULL)
+__global__ void cogroup_count_kernel(u32 nl, u32 nu, u32 lb, const u64 *__restrict__ loffs, const u32 *__restrict__ match,
+                                     const u32 *__restrict__ ronly, const u64 *__restrict__ roffs, int kind,
+                                     u64 *__restrict__ cnt_l, u64 *__restrict__ cnt_r, u64 *__restrict__ cnt_rows)
+{
+    const u32 u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= nu) return;
+    u64 lc, rc;
+    u32 m;
+    cogroup_key(u, nl, lb, loffs, match, ronly, roffs, lc, rc, m);
+    if (cnt_l) cnt_l[u] = lc;
+    if (cnt_r) cnt_r[u] = rc;
+    if (cnt_rows) cnt_rows[u] = (lc && rc) ? lc * rc : lc ? ((kind & CG_LEFT) ? lc : 0) : ((kind & CG_RIGHT) ? rc : 0);
+}
+
+// out[nl + i] = rkeys[ronly[i]]: the right-only keys after the left key slice
+__global__ void cogroup_keys_kernel(const u32 *__restrict__ ronly, u32 nro, const u64 *__restrict__ rkeys, u64 *__restrict__ out)
+{
+    const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < nro) out[i] = rkeys[ronly[i]];
+}
+
+// One thread per right value in union order: binary-search the owning union key in the scanned right counts.
+__global__ void cogroup_gather_right_kernel(const u64 *__restrict__ offs_r /*[nu+1], partition-local*/, u32 nu, u64 total, u32 nl,
+                                            const u32 *__restrict__ match, const u32 *__restrict__ ronly,
+                                            const u64 *__restrict__ roffs, const u64 *__restrict__ rvals, u64 *__restrict__ out)
+{
+    u64 o = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const u64 stride = (u64)gridDim.x * blockDim.x;
+    for (; o < total; o += stride) {
+        const u32 u = cogroup_owner(offs_r, nu, o);
+        const u32 m = u < nl ? match[u] : ronly[u - nl];
+        out[o] = rvals[roffs[m] + (o - offs_r[u])];
+    }
+}
+
+// One thread per outer-join row: binary-search the owning union key, then (v, w) in v-major order; an absent side is
+// written as 0 with its bit clear in valid (1 = v present, 2 = w present).
+__global__ void outer_expand_kernel(const u64 *__restrict__ pos /*[nu] exclusive*/, u32 nu, u64 total, u32 nl, u32 lb,
+                                    const u64 *__restrict__ lkeys, const u64 *__restrict__ loffs, const u64 *__restrict__ lvals,
+                                    const u32 *__restrict__ match, const u32 *__restrict__ ronly, const u64 *__restrict__ rkeys,
+                                    const u64 *__restrict__ roffs, const u64 *__restrict__ rvals, u64 *__restrict__ out_k,
+                                    u64 *__restrict__ out_v, u64 *__restrict__ out_w, unsigned char *__restrict__ out_valid)
+{
+    u64 o = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const u64 stride = (u64)gridDim.x * blockDim.x;
+    for (; o < total; o += stride) {
+        const u32 u = cogroup_owner(pos, nu, o);
+        u64 lc, rc;
+        u32 m;
+        cogroup_key(u, nl, lb, loffs, match, ronly, roffs, lc, rc, m);
+        const u64 local = o - pos[u];
+        u64 v = 0, w = 0;
+        unsigned char valid;
+        if (lc && rc) {
+            const u64 vi = local / rc, wi = local - vi * rc;
+            v = lvals[loffs[lb + u] + vi];
+            w = rvals[roffs[m] + wi];
+            valid = CG_LEFT | CG_RIGHT;
+        } else if (lc) {
+            v = lvals[loffs[lb + u] + local];
+            valid = CG_LEFT;
+        } else {
+            w = rvals[roffs[m] + local];
+            valid = CG_RIGHT;
+        }
+        out_k[o] = u < nl ? lkeys[lb + u] : rkeys[m];
+        out_v[o] = v;
+        out_w[o] = w;
+        if (out_valid) out_valid[o] = valid;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // bincode 1.2.1 blob codec (SURVEY §8(f) N1): pure byte shuffling, HBM-bound
 // ---------------------------------------------------------------------------------------------
 // Vec<(u64,u64)>: out = u64 n | n x (k, c)

@@ -432,20 +432,72 @@ class JoinedRdd(_Base):
         parts = [self.compute(r) for r in range(self.num_slices)]
         return tuple(np.concatenate([p[i] for p in parts]) for i in range(3))
 
+    def cogroup_partition(self, split):
+        """cogroup() of one partition on the device (vb_cogroup): (keys, offs_a, vals_a, offs_b, vals_b).  Keys in union
+        order — this side's keys in its CSR order, then the keys only `other` has; each key's values per side in input
+        order, an empty list on the side that lacks the key.  Offsets are partition-local CSR (n_keys + 1 entries)."""
+        a, b = self._run()
+        lib = self.sc._lib
+        nk, na, nb = ctypes.c_uint64(), ctypes.c_uint64(), ctypes.c_uint64()
+        L.check(lib.vb_cogroup_size(a._h, b._h, split, ctypes.byref(nk), ctypes.byref(na), ctypes.byref(nb)))
+        keys = np.empty(nk.value, dtype=_NP_OF[a.kcode])
+        offs_a = np.empty(nk.value + 1, dtype=np.uint64)
+        offs_b = np.empty(nk.value + 1, dtype=np.uint64)
+        vals_a = np.empty(na.value, dtype=_NP_OF[a.vcode])
+        vals_b = np.empty(nb.value, dtype=_NP_OF[b.vcode])
+        p = lambda x: x.ctypes.data_as(ctypes.c_void_p)
+        L.check(lib.vb_cogroup(a._h, b._h, split, p(keys), p(offs_a), p(vals_a), p(offs_b), p(vals_b), L.VB_HOST))
+        return keys, offs_a, vals_a, offs_b, vals_b
+
     def cogroup_collect(self):
         """cogroup(): per partition, the union of keys with both value lists (co_grouped_rdd.rs:206-249)."""
         a, b = self._run()
         out = []
         for r in range(self.num_slices):
-            ka, oa, va = a.reduce(r)
-            kb, ob, vb = b.reduce(r)
-            g = {}
-            for i, k in enumerate(ka.tolist()):
-                g[k] = [va[int(oa[i]):int(oa[i + 1])], vb[:0]]
-            for i, k in enumerate(kb.tolist()):
-                g.setdefault(k, [va[:0], None])[1] = vb[int(ob[i]):int(ob[i + 1])]
-            out.extend((k, (x[0], x[1])) for k, x in g.items())
+            keys, oa, va, ob, vb = self.cogroup_partition(r)
+            n_left = int(np.count_nonzero(np.diff(oa)))      # union order: every left key has >= 1 left value, the rest none
+            ks = keys[:n_left].tolist() + keys[n_left:].view(_NP_OF[b.kcode]).tolist()
+            oa, ob = oa.tolist(), ob.tolist()
+            out.extend((k, (va[oa[i]:oa[i + 1]], vb[ob[i]:ob[i + 1]])) for i, k in enumerate(ks))
         return out
+
+
+class OuterJoinedRdd(_Base):
+    """`a.left_outer_join(b, n)` / `right_outer_join` / `full_outer_join` (Spark semantics; the reference has no outer
+    joins): the cogroup of both sides, keeping keys that have values on one side only.  Rows of a key are contiguous,
+    keys in the cogroup's union order, `for v in vs { for w in ws }` per matched key."""
+
+    _KINDS = {"left": L.VB_JOIN_LEFT_OUTER, "right": L.VB_JOIN_RIGHT_OUTER, "full": L.VB_JOIN_FULL_OUTER}
+
+    def __init__(self, left, right, num_splits, how):
+        self.joined = JoinedRdd(left, right, num_splits)
+        self.kind = self._KINDS[how]
+        self.num_slices, self.sc = num_splits, left.sc
+
+    def compute(self, split):
+        """(k, v, w, valid): an absent v or w is 0 and its bit (VB_JOIN_HAS_V = 1, VB_JOIN_HAS_W = 2) clear in valid."""
+        a, b = self.joined._run()
+        lib = self.sc._lib
+        n = ctypes.c_uint64()
+        L.check(lib.vb_join_outer_size(a._h, b._h, split, self.kind, ctypes.byref(n)))
+        k = np.empty(n.value, dtype=_NP_OF[a.kcode])
+        v = np.empty(n.value, dtype=_NP_OF[a.vcode])
+        w = np.empty(n.value, dtype=_NP_OF[b.vcode])
+        valid = np.empty(n.value, dtype=np.uint8)
+        p = lambda x: x.ctypes.data_as(ctypes.c_void_p)
+        L.check(lib.vb_join_outer(a._h, b._h, split, self.kind, p(k), p(v), p(w), p(valid), L.VB_HOST))
+        return k, v, w, valid
+
+    def collect(self):
+        parts = [self.compute(r) for r in range(self.num_slices)]
+        return tuple(np.concatenate([p[i] for p in parts]) for i in range(4))
+
+    def to_list(self):
+        """Spark's shape: [(k, (v or None, w or None))]."""
+        k, v, w, valid = self.collect()
+        has_v, has_w = (valid & L.VB_JOIN_HAS_V) != 0, (valid & L.VB_JOIN_HAS_W) != 0
+        return [(kk, (vv if hv else None, ww if hw else None))
+                for kk, vv, ww, hv, hw in zip(k.tolist(), v.tolist(), w.tolist(), has_v.tolist(), has_w.tolist())]
 
 
 class PairRdd(_Base):
@@ -474,6 +526,15 @@ class PairRdd(_Base):
 
     def cogroup(self, other, num_splits):
         return JoinedRdd(self, other, num_splits)
+
+    def left_outer_join(self, other, num_splits):
+        return OuterJoinedRdd(self, other, num_splits, "left")
+
+    def right_outer_join(self, other, num_splits):
+        return OuterJoinedRdd(self, other, num_splits, "right")
+
+    def full_outer_join(self, other, num_splits):
+        return OuterJoinedRdd(self, other, num_splits, "full")
 
     def sort_by_key(self, num_splits):
         return ShuffledRdd(self, "sort", num_splits)
